@@ -2,6 +2,7 @@
 """Benchmark of the VideoPose3D temporal-convolution hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|bf16x3]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -594,6 +595,8 @@ def run_ours(args, rank, local_rank, world):
         torch.cuda.synchronize()
         t_wall = time.perf_counter() - t_wall0
         clocks = sampler.stop()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"pose_3d": y})
         step_ms = [s.elapsed_time(e) for s, e in zip(starts, stops)]
         total_ms = float(sum(step_ms))
         ms = _capi.ctypes.c_float()
@@ -973,6 +976,15 @@ def run_input_pipeline(args):
     return line
 
 
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as `out_dir/<name>.npy` in float32, so that two builds run with the same
+    arguments (hence the same seeded inputs) can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def _visible_index(local_rank):
     vis = os.environ.get("CUDA_VISIBLE_DEVICES", "")
     try:
@@ -984,7 +996,8 @@ def _visible_index(local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 200, or 50 with --input-pipeline)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default="fp16", choices=["fp16", "mixed", "bf16", "bf16x3"])
@@ -999,10 +1012,17 @@ def main():
     ap.add_argument("--input-pipeline", action="store_true",
                     help="measure the training input pipeline (device generator vs CPU port) instead")
     ap.add_argument("--sequences", type=int, default=300)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's prediction (N x 1 x 17 x 3, "
+                         "float32) as DIR/pose_3d.npy")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 50 if args.input_pipeline else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.input_pipeline or args.impl == "reference"):
+        ap.error("--dump-outputs writes the eval forward of --impl ours only")
     if args.input_pipeline:
-        if args.steps == 200:
-            args.steps = 50
         run_input_pipeline(args)
         return
     if args.warmup < 3:
@@ -1023,6 +1043,7 @@ def main():
                "--train-steps", str(args.train_steps), "--sequences", str(args.sequences)]
         cmd += ["--no-train"] if args.no_train else []
         cmd += ["--grad-wire", args.grad_wire] if args.grad_wire else []
+        cmd += ["--dump-outputs", os.path.abspath(args.dump_outputs)] if args.dump_outputs else []
         raise SystemExit(subprocess.call(cmd))
     run_ours(args, rank, local_rank, world)
 

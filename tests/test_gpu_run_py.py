@@ -15,7 +15,13 @@ skipped where neither /root/reference nor the archive exists.  Protocol:
      training kernels: same numbers within bf16 noise;
   5. checkpoint round trip: the epoch-2 checkpoint written by OUR classes is evaluated by the
      reference's classes (`--evaluate`) and vice versa.
+
+Without the reference, test_resume_from_run_py_checkpoint_trains_like_the_reference checks step 3
+against stored reference results (tests/golden/make_run_py_golden.py): training resumed from a
+checkpoint the unchanged run.py wrote, driven as run.py's loop drives it, must reproduce the
+reference's per-step losses and its eval-mode predictions on the trained weights.
 """
+import json
 import os
 import re
 import shutil
@@ -126,3 +132,49 @@ def test_run_py_unchanged_trains_and_evaluates_like_the_reference(tmp_path):
     for k in f_ref:
         assert _close(ev_ref_on_ours[k], f_ours[k], 5e-3), (k, ev_ref_on_ours, f_ours)
         assert _close(ev_ours_on_ref[k], f_ref[k], _tol(k, 5e-3)), (k, ev_ours_on_ref, f_ref)
+
+
+def test_resume_from_run_py_checkpoint_trains_like_the_reference(cuda_device):
+    import numpy as np
+    import videopose3d_b200 as vp
+    from videopose3d_b200 import loss as vloss
+    from videopose3d_b200.optim import FusedAdam
+
+    golden = os.path.join(ROOT, "tests", "golden")
+    sys.path.insert(0, golden)
+    try:
+        import make_run_py_golden as mk
+    finally:
+        sys.path.remove(golden)
+    with open(os.path.join(golden, "run_py_resume.json")) as f:
+        ref = json.load(f)
+    cfg = ref["config"]
+    chk = torch.load(os.path.join(golden, "run_py_epoch_1.bin"), map_location="cpu", weights_only=False)
+    # the fp32-faithful training / inference kernels, as in the run.py comparison above
+    train = vp.TemporalModelOptimized1f(17, 2, 17, filter_widths=cfg["arc"], dropout=0.0,
+                                        channels=cfg["channels"])
+    train.load_state_dict(chk["model_pos"])
+    train = train.to(cuda_device).train().set_train_precision("bf16x3")
+    opt = FusedAdam(train.parameters(), lr=chk["lr"], amsgrad=True)
+    opt.load_state_dict(chk["optimizer"])
+    data, x_eval = mk.batches(cfg)
+    losses = []
+    for x, y in data:
+        opt.zero_grad()
+        loss = vloss.mpjpe(train(x.to(cuda_device)), y.to(cuda_device))
+        loss.backward()
+        opt.step()
+        losses.append(loss.item())
+    ev = vp.TemporalModel(17, 2, 17, filter_widths=cfg["arc"], channels=cfg["channels"])
+    ev.load_state_dict({k: v.cpu() for k, v in train.state_dict().items()})
+    ev = ev.to(cuda_device).eval().set_precision("bf16x3")
+    with torch.no_grad():
+        pred = ev(x_eval.to(cuda_device)).double().cpu().numpy()
+    want = np.array(ref["pred"]).reshape(ref["pred_shape"])
+    print("losses: reference", ref["losses"], "ours", losses)
+    for a, b in zip(ref["losses"], losses):
+        assert _close(a, b, 5e-3), (ref["losses"], losses)
+    assert pred.shape == want.shape
+    err = float(np.abs(pred - want).max() / np.abs(want).max())
+    print(f"eval prediction after {len(losses)} steps: rel err {err:.2e}")
+    assert err <= 5e-3

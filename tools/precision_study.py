@@ -1,5 +1,5 @@
-import sys, torch, numpy as np
-sys.path.insert(0,'/root/repo')
+import os, sys, torch, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import temporal_model_oracle as orc
 torch.set_num_threads(8)
 ARC=[3,3,3,3,3]; C=1024; N=256
